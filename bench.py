@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (one rank per GPU under torchrun)
   python bench.py --impl reference --gpus N --steps K ...  # the CPU path (restated oracle) on the host cores
+  python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   # also write the state after the last timed step as DIR/<field>.npy
 
 A "step" is one mj_step of every environment of the batch (cheetah, 8192 envs per GPU, fresh Philox
 controls every step). `value` is whole-job env-steps/s with inputs resident in HBM; `e2e` is the same
@@ -25,10 +26,16 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
+sys.dont_write_bytecode = True   # the benchmark leaves the source tree as it found it (it may be read-only)
 
 SEED = 0x0B200
 METRIC = "env-steps/sec"
 UNIT = "env-steps/s"
+# --dump-outputs: what a caller reads back after BatchedPhysics.step (fields of size 0 in a model are skipped), at most
+# DUMP_BYTES of array data in all (with the .npy headers, under 64 MB); above that a fixed, seeded sample of environments
+# (the same rows on every run) is written
+DUMP_FIELDS = ("qpos", "qvel", "qacc", "act", "sensordata")
+DUMP_BYTES = 60 << 20
 
 
 def parse_args():
@@ -52,6 +59,8 @@ def parse_args():
     ap.add_argument("--no-spec", action="store_true", help="use the generic fused kernel instead of the model-specialised one")
     ap.add_argument("--ctrl-scale", type=float, default=1.0, help="amplitude of the Philox control stream (power of two; 0.125 = the "
                     "resting-contact regime of the humanoid)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the state after the last timed step as DIR/<field>.npy (batch precision; single rank only)")
     return ap.parse_args()
 
 
@@ -151,6 +160,19 @@ class ClockSampler(threading.Thread):
                 "samples": len(self.samples)}
 
 
+def dump_outputs(b, out_dir, dtype):
+    """Writes DUMP_FIELDS of the batch as out_dir/<field>.npy ([nenv, n] in dtype; [sampled envs, n] above DUMP_BYTES)."""
+    fields = [f for f in DUMP_FIELDS if b.field_size(f) > 0]
+    row_bytes = sum(b.field_size(f) for f in fields) * np.dtype(dtype).itemsize
+    rows = None
+    if row_bytes * b.nenv > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(SEED).choice(b.nenv, DUMP_BYTES // row_bytes, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for f in fields:
+        a = b.get(f, dtype=dtype)
+        np.save(os.path.join(out_dir, f"{f}.npy"), a if rows is None else a[rows])
+
+
 def load_peaks():
     p = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(p):
@@ -209,6 +231,8 @@ def main():
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("bench.py: --dump-outputs applies to the CUDA path only")
         run_reference(args, rank, world)
         return
 
@@ -220,6 +244,8 @@ def main():
 
     if not torch.cuda.is_available():
         raise SystemExit("bench.py: no CUDA device; the product path has no CPU fallback (use --impl reference for the CPU arm)")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("bench.py: --dump-outputs writes one batch; run it with a single rank")
     torch.cuda.set_device(local_rank)
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
@@ -273,6 +299,8 @@ def main():
             evs[i][1].record(stream)
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs:   # before the runs below step the batch further
+        dump_outputs(b, args.dump_outputs, np.float64 if precision == "f64" else np.float32)
     dev_ms = float(sum(s.elapsed_time(e) for s, e in evs))
     launches = b.launch_count() - launches0
     stats = b.stats()
