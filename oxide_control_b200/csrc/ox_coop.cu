@@ -12,14 +12,13 @@
 //     contacts hands item i to lane i % G; tree passes run level by level (parents before children, or children gathered
 //     by their parent - no atomics, deterministic summation order) with a group barrier between levels;
 //   * the dense solves (qacc_smooth = M^-1 f, the Newton step, Euler's implicit damping) are the register-row Cholesky of
-//     the warp solver: lane i owns row i, one shuffle per (column, row) pair;
-//   * the Newton solver is the algorithm of Env::fwd_constraint / k_solve_coop with rows dealt round-robin to lanes.
+//     ox_group_solve.cuh: lane i owns row i, one shuffle per (column, row) pair;
+//   * the Newton solver is group_newton (ox_group_solve.cuh), the one k_solve_coop runs, with rows dealt round-robin to lanes.
 // Generic: any model the compiler accepts with nv <= G, the Newton solver and Euler / implicitfast integration (others keep
 // the thread-per-env kernels). No model-specific code is generated.
-#include <cstdlib>
-
 #include "ox_kernels.cuh"
-#include "ox_spec.cuh"   // StepArgs; pulls in ox_stages.cuh
+#include "ox_group_solve.cuh"
+#include "ox_spec.cuh"   // StepArgs
 
 #ifndef OX_COOP_THREADS
 #define OX_COOP_THREADS 128
@@ -28,7 +27,6 @@
 namespace ox {
 
 constexpr int COOP_THREADS = OX_COOP_THREADS;  // 128: 4 (G = 32) or 8 (G = 16) envs per CTA; the register rows of the dense solves want > 128 registers per thread
-constexpr int CP_SROWS = 32;   // constraint rows of J staged in shared memory for the Hessian build
 
 // ---- per-group shared-memory layout: [DevBatch<T> view][int scalars + body levels][real fields][solver scratch]
 template <typename T>
@@ -52,7 +50,7 @@ OX_HD size_t coop_group_bytes(const CoopSizes<T>& z, int G) {
 #define OX_X(name, cnt) words += (size_t)((cnt) > 0 ? (cnt) : 1);
   OX_BATCH_REAL_FIELDS_SMALL(OX_X)
 #undef OX_X
-  words += (size_t)CP_SROWS * (G + 1) + (size_t)G * (G + 1);
+  words += (size_t)COOP_SROWS * (G + 1) + (size_t)G * (G + 1);
   size_t bytes = sizeof(DevBatch<T>) + (COOP_NINT + (size_t)z.nb) * sizeof(int32_t);
   bytes = (bytes + 15) / 16 * 16 + words * sizeof(T);
   return (bytes + 15) / 16 * 16;
@@ -61,36 +59,26 @@ OX_HD size_t coop_group_bytes(const CoopSizes<T>& z, int G) {
 #if defined(__CUDACC__)
 
 template <typename T, int G>
-struct Coop {
+struct Coop : LaneGroup<G> {
+  using LaneGroup<G>::lane;
+  using LaneGroup<G>::mask;
+  using LaneGroup<G>::sync;
+  using LaneGroup<G>::sum;
   using E = Env<T, DevModel<T>, true>;
   E& env;
-  const int gl;            // lane in group
-  const unsigned gmask;    // lanes of this group within the warp
   int32_t* level;          // [nbody] depth of each body in the tree (world = 0)
   int maxlevel;
-  T* sJ;                   // [CP_SROWS][G + 1]
+  T* sJ;                   // [COOP_SROWS][G + 1]
   T* sL;                   // [G][G + 1]
 
-  __device__ __forceinline__ void gsync() const { __syncwarp(gmask); }
-  __device__ __forceinline__ T gshfl(T v, int src) const { return __shfl_sync(gmask, v, src, G); }
-  __device__ __forceinline__ T gsum(T v) const {
-#pragma unroll
-    for (int o = G / 2; o > 0; o >>= 1) v += __shfl_xor_sync(gmask, v, o, G);
-    return v;
-  }
-  __device__ __forceinline__ int gsumi(int v) const {
-#pragma unroll
-    for (int o = G / 2; o > 0; o >>= 1) v += __shfl_xor_sync(gmask, v, o, G);
-    return v;
-  }
-  __device__ __forceinline__ bool gany(bool p) const { return __ballot_sync(gmask, p) != 0u; }
+  __device__ __forceinline__ bool gany(bool p) const { return __ballot_sync(mask, p) != 0u; }
   // exclusive prefix sum over the lanes of the group
   __device__ __forceinline__ int gscan_excl(int v) const {
     int x = v;
 #pragma unroll
     for (int o = 1; o < G; o <<= 1) {
-      const int y = __shfl_up_sync(gmask, x, o, G);
-      if (gl >= o) x += y;
+      const int y = __shfl_up_sync(mask, x, o, G);
+      if (lane >= o) x += y;
     }
     return x - v;
   }
@@ -100,24 +88,24 @@ struct Coop {
     const auto& m = env.m;
     const int nb = m.h().nbody;
     int mx = 0;
-    for (int i = gl; i < nb; i += G) {
+    for (int i = lane; i < nb; i += G) {
       int d = 0;
       for (int p = i; p > 0; p = m.body_parentid(p)) d++;
       level[i] = d;
       mx = d > mx ? d : mx;
     }
 #pragma unroll
-    for (int o = G / 2; o > 0; o >>= 1) { const int y = __shfl_xor_sync(gmask, mx, o, G); mx = y > mx ? y : mx; }
+    for (int o = G / 2; o > 0; o >>= 1) { const int y = __shfl_xor_sync(mask, mx, o, G); mx = y > mx ? y : mx; }
     maxlevel = mx;
-    gsync();
+    sync();
   }
   // f(i) for every body of each level in turn, parents first
   template <class F> __device__ __forceinline__ void down(int first_level, F f) const {
     const int nb = env.m.h().nbody;
     for (int lv = first_level; lv <= maxlevel; lv++) {
-      for (int i = gl; i < nb; i += G)
+      for (int i = lane; i < nb; i += G)
         if (level[i] == lv) f(i);
-      gsync();
+      sync();
     }
   }
   // field[w*p .. w*p+w) += sum over children c of p (ascending c) of field[w*c ..), deepest parents first; bodies above
@@ -126,7 +114,7 @@ struct Coop {
     const auto& m = env.m;
     const int nb = m.h().nbody;
     for (int lv = maxlevel - 1; lv >= top_level; lv--) {
-      for (int p = gl; p < nb; p += G) {
+      for (int p = lane; p < nb; p += G) {
         if (level[p] != lv) continue;
         T acc[W];
 #pragma unroll
@@ -139,63 +127,11 @@ struct Coop {
 #pragma unroll
         for (int k = 0; k < W; k++) field[W * p + k] = acc[k];
       }
-      gsync();
+      sync();
     }
   }
   template <class F> __device__ __forceinline__ void each(int n, F f) const {
-    for (int i = gl; i < n; i += G) f(i);
-  }
-
-  // ------------------------------------------------------------------ dense Cholesky solve on register rows (lane i = row i)
-  // H (symmetric positive definite, nv x nv): lane i passes row i in Hr[0..nv); returns x_i of H x = rhs. Destroys Hr.
-  __device__ __forceinline__ T chol_solve(T (&Hr)[G], T rhs, int nv) const {
-    T dinv = 1;
-#pragma unroll
-    for (int kk = 0; kk < G; kk++) {
-      if (kk < nv) {  // group-uniform
-        const T piv = gshfl(Hr[kk], kk);
-        const T inv = ox_rsqrt(ox_max(piv, (T)OX_MINVAL));
-        const T lik = Hr[kk] * inv;
-        Hr[kk] = lik;
-        if (gl == kk) dinv = inv;
-#pragma unroll
-        for (int j = kk + 1; j < G; j++) Hr[j] -= lik * gshfl(lik, j);
-      }
-    }
-    T acc = rhs, y = 0;
-#pragma unroll
-    for (int kk = 0; kk < G; kk++) {
-      if (kk < nv) {
-        const T yk = gshfl(acc * dinv, kk);
-        if (gl == kk) y = yk;
-        if (gl > kk) acc -= Hr[kk] * yk;
-      }
-    }
-#pragma unroll
-    for (int j = 0; j < G; j++) sL[gl * (G + 1) + j] = Hr[j];
-    gsync();
-    T x = 0;
-    acc = y;
-    for (int kk = nv - 1; kk >= 0; kk--) {
-      const T xk = gshfl(acc * dinv, kk);
-      if (gl == kk) x = xk;
-      if (gl < kk) acc -= sL[kk * (G + 1) + gl] * xk;
-    }
-    gsync();
-    return x;
-  }
-  // row gl of the dense mass matrix from the sparse qM (0 beyond nv / for idle lanes)
-  __device__ __forceinline__ void load_mrow(T (&Mr)[G]) const {
-    const auto& m = env.m;
-    const int nv = m.h().nv;
-#pragma unroll
-    for (int j = 0; j < G; j++) {
-      Mr[j] = 0;
-      if (j < nv && gl < nv) {
-        const int idx = m.dof_Mdense(gl * nv + j);
-        if (idx >= 0) Mr[j] = env.b.qM[idx];
-      }
-    }
+    for (int i = lane; i < n; i += G) f(i);
   }
 
   // ------------------------------------------------------------------ forward dynamics up to the constraint rows
@@ -212,67 +148,67 @@ struct Coop {
       const T mi = m.body_mass(i);
       for (int k = 0; k < 3; k++) b.subtree_com[3 * i + k] = b.xipos[3 * i + k] * mi;
     });
-    gsync();
+    sync();
     gather_up<3>(b.subtree_com, 0);
     each(nb, [&](int i) {
       const T sm = m.body_subtreemass(i);
       for (int k = 0; k < 3; k++) b.subtree_com[3 * i + k] = sm < (T)OX_MINVAL ? b.xipos[3 * i + k] : b.subtree_com[3 * i + k] / sm;
     });
-    gsync();
+    sync();
     each(nb, [&](int i) {
       if (i == 0) { for (int k = 0; k < 10; k++) b.cinert[k] = 0; } else env.cinert_body(i);
     });
     each(h.njnt, [&](int j) { env.cdof_joint(j); });
-    gsync();
+    sync();
     // composite inertias: own + children, gathered up to the bodies below the world; then one row of M per dof
     each(10 * nb, [&](int k) { b.crb[k] = b.cinert[k]; });
-    gsync();
+    sync();
     gather_up<10>(b.crb, 1);
     each(h.nv, [&](int i) { env.mass_row(i); });
     // narrowphase: one candidate pair per lane, contacts into the static slots of the pair
     each(h.nconmax > 0 ? h.nconmax : 1, [&](int c) { b.con_active[c] = 0; });
-    gsync();
+    sync();
     int mine = 0;
     if (!(env.dis(OX_DSBL_CONTACT) || env.dis(OX_DSBL_CONSTRAINT))) each(h.npair, [&](int p) { env.collide_pair(p, mine); });
-    const int ncon = gsumi(mine);
-    if (gl == 0) b.ncon[0] = ncon;
-    gsync();
+    const int ncon = sum(mine);
+    if (lane == 0) b.ncon[0] = ncon;
+    sync();
   }
   __device__ void fwd_velocity() const {
     const auto& m = env.m;
     const auto& h = m.h();
     const DevBatch<T>& b = env.b;
-    if (gl < 6) b.cvel[gl] = 0;
-    if (gl == 0) {
+    if (lane < 6) b.cvel[lane] = 0;
+    if (lane == 0) {
       T a0[6] = {0, 0, 0, 0, 0, 0};
       if (!env.dis(OX_DSBL_GRAVITY)) { a0[3] = -(T)h.grav(0); a0[4] = -(T)h.grav(1); a0[5] = -(T)h.grav(2); }
       for (int k = 0; k < 6; k++) { b.cacc[k] = a0[k]; b.cfrc[k] = 0; }
     }
     each(h.nv, [&](int i) { b.qfrc_passive[i] = 0; });
     each(h.ntendon, [&](int i) { env.tendon_length(i); });
-    gsync();
+    sync();
     down(1, [&](int i) { env.vel_body(i); });
     if (!env.dis(OX_DSBL_PASSIVE)) {
       each(h.njnt, [&](int j) { env.passive_joint(j); });
-      gsync();
+      sync();
       each(h.nv, [&](int i) { b.qfrc_passive[i] -= m.dof_damping(i) * b.qvel[i]; });
       if (h.ntendon > 0) {   // a tendon touches several dofs: one lane applies them in order
-        gsync();
-        if (gl == 0) for (int i = 0; i < h.ntendon; i++) env.passive_tendon(i);
+        sync();
+        if (lane == 0) for (int i = 0; i < h.ntendon; i++) env.passive_tendon(i);
       }
       if (h.nfluid > 0) {    // fluid drag: a body's wrench touches its whole dof chain, same rule
-        gsync();
-        if (gl == 0) for (int bd = 1; bd < h.nfluid; bd++) env.passive_fluid(bd);
+        sync();
+        if (lane == 0) for (int bd = 1; bd < h.nfluid; bd++) env.passive_fluid(bd);
       }
       if (h.ngravcomp > 0 && !env.dis(OX_DSBL_GRAVITY)) {
-        gsync();
-        if (gl == 0) for (int bd = 1; bd < h.ngravcomp; bd++) env.passive_gravcomp(bd);
+        sync();
+        if (lane == 0) for (int bd = 1; bd < h.ngravcomp; bd++) env.passive_gravcomp(bd);
       }
     }
     down(1, [&](int i) { env.rne_fwd_body(i); });
     gather_up<6>(b.cfrc, 1);
     each(h.nv, [&](int i) { env.rne_bias_dof(i); });
-    gsync();
+    sync();
   }
   // constraint rows: counts per item, exclusive scan across the group, rows written in place - same row order as the serial code
   __device__ void make_constraint() const {
@@ -283,32 +219,32 @@ struct Coop {
     if (!env.dis(OX_DSBL_CONSTRAINT)) {
       if (!env.dis(OX_DSBL_EQUALITY)) {
         for (int i0 = 0; i0 < h.neq; i0 += G) {
-          const int i = i0 + gl;
+          const int i = i0 + lane;
           const int cnt = i < h.neq ? env.equality_count(i) : 0;
           int r = base + gscan_excl(cnt);
           if (cnt) env.equality_rows(i, r);
-          base += gsumi(cnt);
+          base += sum(cnt);
         }
       }
-      if (gl == 0) b.ne[0] = base;
+      if (lane == 0) b.ne[0] = base;
       if (!env.dis(OX_DSBL_LIMIT)) {
         for (int j0 = 0; j0 < h.njnt; j0 += G) {
-          const int j = j0 + gl;
+          const int j = j0 + lane;
           const int cnt = j < h.njnt ? env.limit_count(j) : 0;
           int r = base + gscan_excl(cnt);
           if (cnt) env.limit_rows(j, r);
-          base += gsumi(cnt);
+          base += sum(cnt);
         }
         for (int i0 = 0; i0 < h.ntendon; i0 += G) {
-          const int i = i0 + gl;
+          const int i = i0 + lane;
           const int cnt = i < h.ntendon ? env.tendon_limit_count(i) : 0;
           int r = base + gscan_excl(cnt);
           if (cnt) env.tendon_limit_rows(i, r);
-          base += gsumi(cnt);
+          base += sum(cnt);
         }
       }
       for (int c0 = 0; c0 < h.nconmax; c0 += G) {
-        const int c = c0 + gl;
+        const int c = c0 + lane;
         int cnt = 0, p = 0;
         if (c < h.nconmax && b.con_active[c]) {
           p = b.con_pair[c];
@@ -317,18 +253,18 @@ struct Coop {
         }
         int r = base + gscan_excl(cnt);
         if (cnt) env.contact_rows(c, p, r);
-        base += gsumi(cnt);
+        base += sum(cnt);
       }
     }
-    if (gl == 0) { b.nefc[0] = base; if (env.dis(OX_DSBL_CONSTRAINT)) b.ne[0] = 0; }
-    gsync();
+    if (lane == 0) { b.nefc[0] = base; if (env.dis(OX_DSBL_CONSTRAINT)) b.ne[0] = 0; }
+    sync();
   }
   __device__ void actuation_and_smooth() const {
     const auto& m = env.m;
     const auto& h = m.h();
     const DevBatch<T>& b = env.b;
     each(h.nu, [&](int i) { (void)env.actuator_one(i); });
-    gsync();
+    sync();
     each(h.nv, [&](int d) {   // gather the actuators of this dof in index order (several may drive one joint)
       T f = 0;
       if (!env.dis(OX_DSBL_ACTUATION))
@@ -337,204 +273,24 @@ struct Coop {
       b.qfrc_actuator[d] = f;
       b.qfrc_smooth[d] = b.qfrc_passive[d] - b.qfrc_bias[d] + b.qfrc_applied[d] + f;
     });
-    gsync();
+    sync();
     if (applied) {
-      if (gl == 0) env.apply_xfrc();
-      gsync();
+      if (lane == 0) env.apply_xfrc();
+      sync();
     }
     T Mr[G];
-    load_mrow(Mr);
-    const T as = chol_solve(Mr, gl < h.nv ? b.qfrc_smooth[gl] : (T)0, h.nv);
-    if (gl < h.nv) b.qacc_smooth[gl] = as;
-    gsync();
+    group_load_mrow(*this, m, b.qM, ElemAt{1, 0}, Mr);
+    const T as = group_chol_solve(*this, Mr, lane < h.nv ? b.qfrc_smooth[lane] : (T)0, h.nv, sL);
+    if (lane < h.nv) b.qacc_smooth[lane] = as;
+    sync();
   }
   int applied = 1;
 
-  // ------------------------------------------------------------------ Newton solver (Env::fwd_constraint, rows over lanes)
-  __device__ void solve() const {
-    const auto& m = env.m;
-    const auto& h = m.h();
-    const DevBatch<T>& b = env.b;
-    const int nv = h.nv, nefc = b.nefc[0], ne = b.ne[0];   // rows below ne are equality rows: active on both sides
-    const bool me = gl < nv;
-    if (nefc == 0) {
-      if (me) { const T a = b.qacc_smooth[gl]; b.qacc[gl] = a; b.qacc_warmstart[gl] = a; b.qfrc_constraint[gl] = 0; }
-      if (gl == 0) b.solver_niter[0] = 0;
-      gsync();
-      return;
-    }
-    T* rowD = b.efc_D; T* rowA = b.efc_aref; T* rowJar = b.s_Jaref; T* rowJv = b.s_Jv; T* rowF = b.efc_force;
-    const T* J = b.efc_J;
-    const int nsm = nefc < CP_SROWS ? nefc : CP_SROWS;
-    for (int r = 0; r < nsm; r++) sJ[r * (G + 1) + gl] = me ? J[r * nv + gl] : (T)0;
-    gsync();
-    auto Jat = [&](int r, int i) -> T { return r < CP_SROWS ? sJ[r * (G + 1) + i] : J[r * nv + i]; };
-    const T fs = me ? b.qfrc_smooth[gl] : (T)0, as = me ? b.qacc_smooth[gl] : (T)0, aw = me ? b.qacc_warmstart[gl] : (T)0;
-    T Mrow[G];
-    load_mrow(Mrow);
-    auto Mdot = [&](T x) -> T {
-      T acc = 0;
-#pragma unroll
-      for (int j = 0; j < G; j++)
-        if (j < nv) acc += Mrow[j] * gshfl(x, j);
-      return acc;
-    };
-    auto Jdot = [&](T x, T* out, bool minus_aref) {
-      for (int r0 = 0; r0 < nefc; r0 += G) {
-        const int r = r0 + gl;
-        T acc = 0;
-#pragma unroll 4
-        for (int i = 0; i < nv; i++) {
-          const T xi = gshfl(x, i);
-          if (r < nefc) acc += Jat(r, i) * xi;
-        }
-        if (r < nefc) out[r] = minus_aref ? acc - rowA[r] : acc;
-      }
-      gsync();
-    };
-    bool use_smooth = true;
-    if (!(h.disableflags & OX_DSBL_WARMSTART)) {
-      T cand[2];
-#pragma unroll 1
-      for (int c = 0; c < 2; c++) {
-        const T x = c ? as : aw;
-        const T Mx = Mdot(x);
-        T cc = me ? (T)0.5 * (Mx - fs) * (x - as) : (T)0;
-        Jdot(x, rowJv, true);
-        for (int r = gl; r < nefc; r += G) {
-          const T v = rowJv[r];
-          if (v < 0 || r < ne) cc += (T)0.5 * rowD[r] * v * v;
-        }
-        cand[c] = gsum(cc);
-        gsync();
-      }
-      use_smooth = cand[0] > cand[1];
-    }
-    T a = use_smooth ? as : aw;
-    T Ma = Mdot(a);
-    Jdot(a, rowJar, true);
-    T fc = 0, gauss = 0, cost = 0, grad = 0, Mgrad = 0, gnorm = 0, search = 0;
-    const T tol = (T)h.tolerance;
-    const T mscale = (T)h.meaninertia * (T)(nv > 1 ? nv : 1);
-    const T scale = (T)1 / mscale;
-    const int maxiter = h.iterations;
-    int iter = 0;
-    bool init = true;
-#pragma unroll 1
-    for (;;) {
-      if (!init) {
-        if (iter >= maxiter) break;
-        const T snorm = ox_sqrt(gsum(search * search));
-        if (snorm < (T)OX_MINVAL) break;
-        const T gtol = tol * (T)h.ls_tolerance * snorm * mscale;
-        const T Mv = Mdot(search);
-        Jdot(search, rowJv, false);
-        const T qg1 = gsum(me ? search * (Ma - fs) : (T)0), qg2 = gsum(me ? (T)0.5 * search * Mv : (T)0);
-        T p0c = 0, p0d0 = 0, cur_a = 0, cur_c = 0, cur_d0 = 0, cur_d1 = 1, lo_a = 0, hi_a = 0;
-        bool have_hi = false, stop = false;
-#pragma unroll 1
-        for (int it = -1; it < h.ls_iterations && !stop; it++) {
-          T an = 0;
-          if (it >= 0) {
-            an = cur_a - cur_d0 / cur_d1;
-            if (have_hi && !(an > lo_a && an < hi_a)) an = (T)0.5 * (lo_a + hi_a);
-            if (ox_abs(an - cur_a) <= Eps<T>::v() * ox_abs(an)) break;
-          }
-          T c = 0, d0 = 0, d1 = 0, s0 = 0;
-          for (int r = gl; r < nefc; r += G) {
-            const T ja = rowJar[r], jvr = rowJv[r];
-            const T x = ja + an * jvr;
-            if (x < 0 || r < ne) {
-              const T Dx = rowD[r] * x, Dj = rowD[r] * jvr;
-              c += (T)0.5 * Dx * x;
-              d0 += Dx * jvr;
-              d1 += Dj * jvr;
-              s0 += ox_abs(Dx * jvr);
-            }
-          }
-          cur_a = an;
-          cur_c = an * an * qg2 + an * qg1 + gauss + gsum(c);
-          cur_d0 = 2 * an * qg2 + qg1 + gsum(d0);
-          cur_d1 = 2 * qg2 + gsum(d1);
-          const T cur_s0 = ox_abs(2 * an * qg2) + ox_abs(qg1) + gsum(s0);
-          if (cur_d1 < (T)OX_MINVAL) cur_d1 = (T)OX_MINVAL;
-          if (it < 0) {
-            p0c = cur_c; p0d0 = cur_d0;
-            if (!(p0d0 < 0)) stop = true;
-          } else {
-            if (ox_abs(cur_d0) < gtol || ox_abs(cur_d0) <= 8 * Eps<T>::v() * cur_s0) break;
-            if (cur_d0 < 0) lo_a = cur_a; else { hi_a = cur_a; have_hi = true; }
-          }
-        }
-        if (stop) break;
-        const T alpha = cur_c <= p0c ? cur_a : (T)0;
-        if (alpha == 0) break;
-        a += alpha * search;
-        Ma += alpha * Mv;
-        for (int r = gl; r < nefc; r += G) rowJar[r] += alpha * rowJv[r];
-        gsync();
-      }
-      const T oldcost = cost;
-      {
-        T crow = 0;
-        for (int r = gl; r < nefc; r += G) {
-          const T ja = rowJar[r];
-          T f = 0;
-          if (ja < 0 || r < ne) { f = -rowD[r] * ja; crow += (T)0.5 * rowD[r] * ja * ja; }
-          rowF[r] = f;
-        }
-        gsync();
-        fc = 0;
-        for (int r = 0; r < nefc; r++) {
-          const T f = rowF[r];
-          if (f != 0 && me) fc += Jat(r, gl) * f;
-        }
-        gauss = gsum(me ? (T)0.5 * (Ma - fs) * (a - as) : (T)0);
-        cost = gsum(crow) + gauss;
-      }
-      {
-        grad = me ? Ma - fs - fc : (T)0;
-        gnorm = ox_sqrt(gsum(grad * grad));
-        T Hreg[G];
-#pragma unroll
-        for (int j = 0; j < G; j++) Hreg[j] = Mrow[j];
-        for (int r = 0; r < nefc; r++) {
-          if (!(rowJar[r] < 0 || r < ne)) continue;  // group-uniform
-          if (r < CP_SROWS) {
-            const T* jr = sJ + r * (G + 1);
-            const T s = rowD[r] * jr[gl];
-#pragma unroll
-            for (int j = 0; j < G; j++) Hreg[j] += s * jr[j];
-          } else {
-            const T Jri = me ? J[r * nv + gl] : (T)0;
-            const T s = rowD[r] * Jri;
-#pragma unroll
-            for (int j = 0; j < G; j++) Hreg[j] += s * gshfl(Jri, j);
-          }
-        }
-        Mgrad = chol_solve(Hreg, grad, nv);
-      }
-      if (init) {
-        init = false;
-        if (scale * gnorm < tol) break;
-      } else {
-        iter++;
-        const T improvement = scale * (oldcost - cost), gradient = scale * gnorm;
-        if (improvement < tol || gradient < tol) break;
-        if (oldcost - cost <= OX_FLOOR_MULT * Eps<T>::v() * (ox_abs(oldcost) + ox_abs(cost))) break;
-      }
-      search = -Mgrad;
-    }
-    if (me) { b.qacc[gl] = a; b.qacc_warmstart[gl] = a; b.qfrc_constraint[gl] = fc; }
-    if (gl == 0) b.solver_niter[0] = iter;
-    gsync();
-  }
-
-  // CTA-wide barrier between stages (lockstep != 0): the 4 warps of a CTA then stream the same part of the ~700 KB body at
-  // the same time and share its instruction-cache fills, at the price of waiting for the slowest env of the CTA in the solver
-  int lockstep = 0;
   bool live = true;   // false: a group of the tail CTA beyond nenv - it only keeps the CTA barriers company
-  __device__ __forceinline__ void stage_barrier() const { if (lockstep) __syncthreads(); }
+  // CTA-wide barrier between stages: the warps of a CTA then stream the same part of the ~700 KB body at the same time and
+  // share its instruction-cache fills, at the price of waiting for the slowest env of the CTA in the solver (humanoid 4096
+  // envs: 1.19 -> 0.90 ms per step, 300 steps in one launch 2.5 x faster than without)
+  __device__ __forceinline__ void stage_barrier() const { __syncthreads(); }
   __device__ void forward(bool skipsensor) const {
     if (live) fwd_position();
     stage_barrier();
@@ -544,11 +300,11 @@ struct Coop {
     stage_barrier();
     if (live) actuation_and_smooth();
     stage_barrier();
-    if (live) solve();
+    if (live) group_newton<T, G, 0>(*this, env.m, env.b, ElemAt{1, 0}, sJ, sL, nullptr);   // per-row scalars stay in the arena
     stage_barrier();
     if (live && !skipsensor && env.m.h().nsensor > 0) {
-      if (gl == 0) env.sensors();
-      gsync();
+      if (lane == 0) env.sensors();
+      sync();
     }
   }
 
@@ -568,8 +324,8 @@ struct Coop {
     return gany(bad);
   }
   __device__ void reset() const {
-    if (gl == 0) { env.reset_data(); env.b.diverged[0] += 1; }
-    gsync();
+    if (lane == 0) { env.reset_data(); env.b.diverged[0] += 1; }
+    sync();
   }
   __device__ void euler() const {
     const auto& m = env.m;
@@ -578,14 +334,14 @@ struct Coop {
     const int nv = h.nv;
     const bool fast = h.integrator == OX_INT_IMPLICITFAST;
     const T dt = (T)h.timestep;
-    T qa = gl < nv ? b.qacc[gl] : (T)0;
+    T qa = lane < nv ? b.qacc[lane] : (T)0;
     if (fast || (h.any_damping && !env.dis(OX_DSBL_EULERDAMP))) {
       // (M + h B) qacc' = qfrc_smooth + qfrc_constraint, B as in Env::euler (joint damping; implicitfast: - actuator velocity derivative)
-      T d = gl < nv ? dt * m.dof_damping(gl) : (T)0;
-      if (fast && !env.dis(OX_DSBL_ACTUATION) && gl < nv) {
+      T d = lane < nv ? dt * m.dof_damping(lane) : (T)0;
+      if (fast && !env.dis(OX_DSBL_ACTUATION) && lane < nv) {
         const bool clamp = !env.dis(OX_DSBL_CLAMPCTRL);
         for (int i = 0; i < h.nu; i++) {
-          if (m.jnt_dofadr(m.actuator_trnid(i)) != gl) continue;
+          if (m.jnt_dofadr(m.actuator_trnid(i)) != lane) continue;
           const bool gaff = m.actuator_gaintype(i) == OX_GAIN_AFFINE, baff = m.actuator_biastype(i) == OX_BIAS_AFFINE;
           if (!gaff && !baff) continue;
           if (m.actuator_forcelimited(i)) {
@@ -600,11 +356,11 @@ struct Coop {
         }
       }
       T Hr[G];
-      load_mrow(Hr);
+      group_load_mrow(*this, m, b.qM, ElemAt{1, 0}, Hr);
 #pragma unroll
       for (int j = 0; j < G; j++)
-        if (j == gl) Hr[j] += d;   // static register indices only (a runtime index would push the row into local memory)
-      qa = chol_solve(Hr, gl < nv ? b.qfrc_smooth[gl] + b.qfrc_constraint[gl] : (T)0, nv);
+        if (j == lane) Hr[j] += d;   // static register indices only (a runtime index would push the row into local memory)
+      qa = group_chol_solve(*this, Hr, lane < nv ? b.qfrc_smooth[lane] + b.qfrc_constraint[lane] : (T)0, nv, sL);
     }
     // mj_advance: activations, velocities, then positions with the new velocities, time
     each(h.nu, [&](int i) {
@@ -612,11 +368,11 @@ struct Coop {
       const int aa = m.actuator_actadr(i);
       b.act[aa] = env.next_activation(i, b.act[aa], b.act_dot[aa]);
     });
-    if (gl < nv) b.qvel[gl] += dt * qa;
-    gsync();
+    if (lane < nv) b.qvel[lane] += dt * qa;
+    sync();
     each(h.njnt, [&](int j) { env.integrate_pos_joint(b.qpos, b.qvel, dt, j); });
-    if (gl == 0) b.time[0] += dt;
-    gsync();
+    if (lane == 0) b.time[0] += dt;
+    sync();
   }
   __device__ void step() const {
     if (live && bad_state()) reset();
@@ -625,12 +381,12 @@ struct Coop {
       forward(false);
       // (with CTA barriers inside forward() every group of the CTA must take the same number of passes)
       const bool mine = live && bad_acc();
-      const bool redo = !pass && (lockstep ? __syncthreads_or(mine) != 0 : mine);
+      const bool redo = !pass && __syncthreads_or(mine) != 0;
       if (!redo) break;
       if (mine) reset();
     }
     if (!live) return;
-    if (gl == 0) env.accumulate_stats();
+    if (lane == 0) env.accumulate_stats();
     euler();
   }
 };
@@ -642,10 +398,7 @@ __global__ void __launch_bounds__(COOP_THREADS, COOP_THREADS >= 256 ? 1 : 2) k_s
   constexpr int GPC = COOP_THREADS / G;
   const int gic = threadIdx.x / G, gl = threadIdx.x % G;
   const int e_raw = blockIdx.x * GPC + gic;
-  const bool lockstep = group_bytes < 0;      // sign bit of the argument carries the launch option
-  if (lockstep) group_bytes = -group_bytes;
-  if (!lockstep && e_raw >= g.nenv) return;
-  const bool live = e_raw < g.nenv;            // lockstep: the spare groups of a tail CTA do no work but join the CTA barriers
+  const bool live = e_raw < g.nenv;            // the spare groups of a tail CTA do no work but join the CTA barriers
   const int e = live ? e_raw : g.nenv - 1;
   const unsigned gmask = G == 32 ? 0xffffffffu : (((1u << G) - 1u) << (((threadIdx.x & 31) / G) * G));
   const BlobHeader& h = m.h();
@@ -683,9 +436,8 @@ __global__ void __launch_bounds__(COOP_THREADS, COOP_THREADS >= 256 ? 1 : 2) k_s
   }
   Env<T, DevModel<T>, true> env(m, *lb, 0);
   env.slots = true;
-  Coop<T, G> c{env, gl, gmask, ib + COOP_NINT, 0, scratch, scratch + CP_SROWS * (G + 1)};
+  Coop<T, G> c{{gl, gmask}, env, ib + COOP_NINT, 0, scratch, scratch + COOP_SROWS * (G + 1)};
   c.applied = a.applied;
-  c.lockstep = lockstep ? 1 : 0;
   c.live = live;
   c.compute_levels();
   const DevBatch<T>& b = *lb;
@@ -711,7 +463,8 @@ __global__ void __launch_bounds__(COOP_THREADS, COOP_THREADS >= 256 ? 1 : 2) k_s
   const int32_t div0 = b.diverged[0];
   const long long step0 = a.d_step ? *a.d_step : a.step0;
   for (int s = 0; s < a.nsteps; s++) {
-    if (a.philox && live) {
+    // a spare group fills its own view too (never written back): a `live` test here costs k_step_coop<double, 32> a spill
+    if (a.philox) {
       if (gl == 0) env.fill_ctrl_philox(a.seed, a.env_id_offset + e, step0 + s, (T)a.ctrl_scale);
       __syncwarp(gmask);
     }
@@ -777,12 +530,8 @@ static cudaError_t launch_coop_step(cudaStream_t stream, const ox_model_tables& 
   const int gpc = COOP_THREADS / G, grid = (g.nenv + gpc - 1) / gpc;
   const size_t gb = coop_group_bytes_host<T>(t, G);
   const size_t smem = (size_t)((bytes + 127) / 128) * 128 + (size_t)gpc * gb;
-  // CTA barriers between stages are on by default (humanoid 4096 envs: 1.19 -> 0.90 ms per step, 300 steps in one launch
-  // 2.5 x faster); OX_B200_COOP_LOCKSTEP=0 turns them off for A/B measurements
-  static const bool lockstep = [] { const char* v = getenv("OX_B200_COOP_LOCKSTEP"); return !(v && v[0] == '0'); }();
-  const int gba = lockstep ? -(int)gb : (int)gb;
-  if (G == 16) k_step_coop<T, 16><<<grid, COOP_THREADS, smem, stream>>>(blob, bytes, g, a, gba);
-  else k_step_coop<T, 32><<<grid, COOP_THREADS, smem, stream>>>(blob, bytes, g, a, gba);
+  if (G == 16) k_step_coop<T, 16><<<grid, COOP_THREADS, smem, stream>>>(blob, bytes, g, a, (int)gb);
+  else k_step_coop<T, 32><<<grid, COOP_THREADS, smem, stream>>>(blob, bytes, g, a, (int)gb);
   return cudaPeekAtLastError();
 }
 cudaError_t launch_step_coop_f32(cudaStream_t s, const ox_model_tables& t, const unsigned char* blob, int bytes, const DevBatch<float>& g, const StepArgs& a) { return launch_coop_step<float>(s, t, blob, bytes, g, a); }

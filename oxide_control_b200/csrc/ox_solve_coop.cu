@@ -1,297 +1,19 @@
 // Warp-cooperative primal Newton solver (mj_fwdConstraint / mj_solNewton; SURVEY.md A.11): ONE WARP PER ENVIRONMENT,
 // lane = dof. It replaces the thread-per-env solve stage for models whose constraint problem is too large to sit in
 // one thread's registers (humanoid class: nv = 27, H = 27x27): there the serial solve is >90 % of the step and the GPU
-// holds only nenv/32 warps. Here
-//   * every dof-vector (qacc, M*qacc, grad, search, ...) is one register per lane,
-//   * lane i owns row i of the dense Hessian H = M + J' D J in 32 registers: the rank-1 row updates read the staged J
-//     row with broadcast shared-memory loads, the right-looking Cholesky exchanges one shuffle per (column, row) pair,
-//     the triangular solves one shuffle / butterfly per column. Only this block is unrolled (about 3 k instructions, one
-//     call site); v1 unrolled everything at three call sites (34 k instructions, `no_instruction` 10.7 cycles per issue -
-//     profiles/r1_ncu_coop_v1_humanoid_f32_4096.txt), v2/v3 kept H in shared memory (4 instructions and a shared-memory
-//     round trip per multiply-add); M's row also stays in registers,
-//   * constraint rows are distributed round-robin over lanes (row r -> lane r % 32) for jar / Jv / line search, their
-//     per-row scalars in per-warp shared arrays,
-//   * the active part of J is staged once per solve into shared memory ([row][dof], padded) because the batch stores it
-//     [element][env] (lane = env layout), which this kernel can only gather from.
-// Same algorithm, stopping rules and warm start as Env::fwd_constraint (ox_stages.cuh); only the summation order differs.
+// holds only nenv/32 warps. The solve itself is group_newton (ox_group_solve.cuh) with G = 32; this kernel gives each
+// warp shared-memory scratch for it, including per-row scalar arrays for envs with at most COOP_RCAP rows.
 // Eligibility (checked on the host): Newton solver, nv <= 32.
-#include <cstdlib>
-
 #include "ox_kernels.cuh"
-#include "ox_stages.cuh"
+#include "ox_group_solve.cuh"
 
 namespace ox {
 
-constexpr int COOP_SROWS = 32;     // rows of J staged in shared memory per warp; the rest is read from the arena
 constexpr int COOP_WARPS = 8;      // warps (= consecutive envs) per CTA: their gathers from the [element][env] arena share 32-byte sectors
 constexpr int COOP_RCAP = 96;      // rows whose per-row scalars live in shared memory; envs with more rows use the arena's row arrays
 
-template <typename T> __device__ __forceinline__ T wsum(T v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  return v;
-}
-template <typename T> __device__ __forceinline__ T bcast(T v, int src) { return __shfl_sync(0xffffffffu, v, src); }
-__device__ __forceinline__ float coop_rsqrt(float x) { return rsqrtf(x); }
-__device__ __forceinline__ double coop_rsqrt(double x) { return rsqrt(x); }
-
 // per-warp shared memory: five row arrays of RCAP, J staging (SROWS x 33), the Cholesky factor (32 x 33) for the back substitution
 __host__ __device__ inline size_t coop_warp_words() { return 5 * (size_t)COOP_RCAP + COOP_SROWS * 33 + 32 * 33; }
-
-// one environment's solve by one warp (the body of the kernel below)
-template <typename T>
-__device__ __forceinline__ void coop_solve_env(const DevModel<T>& m, const DevBatch<T>& b, unsigned char* ox_smem, int bytes, int env, int wib, int lane) {
-  const BlobHeader& h = m.h();
-  const int nv = h.nv;
-  const bool me = lane < nv;
-  const uint32_t S = (uint32_t)b.stride, ue = (uint32_t)env;
-#define GA(field, i) b.field[(uint32_t)(i) * S + ue]
-  const int nefc = b.nefc[ue], ne = b.ne[ue];   // rows below ne are equality rows: active on both sides
-  if (nefc == 0) {
-    if (me) {
-      const T a = GA(qacc_smooth, lane);
-      GA(qacc, lane) = a; GA(qacc_warmstart, lane) = a; GA(qfrc_constraint, lane) = 0;
-    }
-    if (lane == 0) b.solver_niter[ue] = 0;
-    return;
-  }
-  T* srow = reinterpret_cast<T*>(ox_smem + ((bytes + 127) / 128) * 128) + (size_t)wib * coop_warp_words();
-  T* sJ = srow + 5 * COOP_RCAP;
-  T* sL = sJ + COOP_SROWS * 33;
-  // per-row scalars: shared memory (stride 1) for the common case, the arena's own row arrays (stride S) when an env has
-  // more rows than RCAP. efc_D / efc_aref are then read in place; jar, Jv and force use s_Jaref, s_Jv, efc_force.
-  const bool small = nefc <= COOP_RCAP;
-  const uint32_t rs = small ? 1u : S;
-  T* rowD = small ? srow : b.efc_D + ue;
-  T* rowA = small ? rowD + COOP_RCAP : b.efc_aref + ue;
-  T* rowJar = small ? rowA + COOP_RCAP : b.s_Jaref + ue;
-  T* rowJv = small ? rowJar + COOP_RCAP : b.s_Jv + ue;
-  T* rowF = small ? rowJv + COOP_RCAP : b.efc_force + ue;
-#define ROW(arr, r) arr[(uint32_t)(r) * rs]
-  const int nsm = nefc < COOP_SROWS ? nefc : COOP_SROWS;
-  for (int r = 0; r < nsm; r++)
-    sJ[r * 33 + lane] = me ? GA(efc_J, r * nv + lane) : (T)0;
-  if (small)
-    for (int r = lane; r < nefc; r += 32) { rowD[r] = GA(efc_D, r); rowA[r] = GA(efc_aref, r); }
-  __syncwarp();
-  auto Jat = [&](int r, int i) -> T { return r < COOP_SROWS ? sJ[r * 33 + i] : GA(efc_J, r * nv + i); };
-
-  const T fs = me ? GA(qfrc_smooth, lane) : (T)0, as = me ? GA(qacc_smooth, lane) : (T)0, aw = me ? GA(qacc_warmstart, lane) : (T)0;
-  // dense row `lane` of the mass matrix, in registers (static indices only)
-  T Mrow[32];
-#pragma unroll
-  for (int j = 0; j < 32; j++) {
-    Mrow[j] = 0;
-    if (j < nv && me) {
-      const int idx = m.dof_Mdense(lane * nv + j);
-      if (idx >= 0) Mrow[j] = GA(qM, idx);
-    }
-  }
-  auto Mdot = [&](T x) -> T {  // (M x)_lane, x distributed one element per lane
-    T acc = 0;
-#pragma unroll
-    for (int j = 0; j < 32; j++)
-      if (j < nv) acc += Mrow[j] * bcast(x, j);
-    return acc;
-  };
-  auto Jdot = [&](T x, T* out, bool minus_aref) {  // out[r] = J_r . x (- aref_r), rows round-robin over lanes
-    for (int r0 = 0; r0 < nefc; r0 += 32) {
-      const int r = r0 + lane;
-      T acc = 0;
-#pragma unroll 4
-      for (int i = 0; i < nv; i++) {
-        const T xi = bcast(x, i);
-        if (r < nefc) acc += Jat(r, i) * xi;
-      }
-      if (r < nefc) ROW(out, r) = minus_aref ? acc - ROW(rowA, r) : acc;
-    }
-    __syncwarp();
-  };
-
-  // warm start: cheaper of cost(qacc_warmstart), cost(qacc_smooth), through one evaluation site
-  bool use_smooth = true;
-  if (!(h.disableflags & OX_DSBL_WARMSTART)) {
-    T cand[2];
-#pragma unroll 1
-    for (int c = 0; c < 2; c++) {
-      const T x = c ? as : aw;
-      const T Mx = Mdot(x);
-      T cc = me ? (T)0.5 * (Mx - fs) * (x - as) : (T)0;
-      Jdot(x, rowJv, true);
-      for (int r = lane; r < nefc; r += 32) {
-        const T v = ROW(rowJv, r);
-        if (v < 0 || r < ne) cc += (T)0.5 * ROW(rowD, r) * v * v;
-      }
-      cand[c] = wsum(cc);
-      __syncwarp();
-    }
-    use_smooth = cand[0] > cand[1];
-  }
-  T a = use_smooth ? as : aw;
-  T Ma = Mdot(a);
-  Jdot(a, rowJar, true);
-
-  T fc = 0, gauss = 0, cost = 0, grad = 0, Mgrad = 0, gnorm = 0, search = 0;
-  const T tol = (T)h.tolerance;
-  const T mscale = (T)h.meaninertia * (T)(nv > 1 ? nv : 1);
-  const T scale = (T)1 / mscale;
-  const int maxiter = h.iterations;
-  int iter = 0;
-  bool init = true;
-#pragma unroll 1
-  for (;;) {
-    if (!init) {
-      if (iter >= maxiter) break;
-      // ---- exact line search on the convex piecewise-quadratic phi(alpha)
-      const T snorm = ox_sqrt(wsum(search * search));
-      if (snorm < (T)OX_MINVAL) break;
-      const T gtol = tol * (T)h.ls_tolerance * snorm * mscale;
-      const T Mv = Mdot(search);
-      Jdot(search, rowJv, false);
-      const T qg1 = wsum(me ? search * (Ma - fs) : (T)0), qg2 = wsum(me ? (T)0.5 * search * Mv : (T)0);
-      T p0c = 0, p0d0 = 0, cur_a = 0, cur_c = 0, cur_d0 = 0, cur_d1 = 1, lo_a = 0, hi_a = 0;
-      bool have_hi = false, stop = false;
-#pragma unroll 1
-      for (int it = -1; it < h.ls_iterations && !stop; it++) {  // it = -1 evaluates alpha = 0
-        T an = 0;
-        if (it >= 0) {
-          an = cur_a - cur_d0 / cur_d1;
-          if (have_hi && !(an > lo_a && an < hi_a)) an = (T)0.5 * (lo_a + hi_a);
-          if (ox_abs(an - cur_a) <= Eps<T>::v() * ox_abs(an)) break;
-        }
-        T c = 0, d0 = 0, d1 = 0, s0 = 0;
-        for (int r = lane; r < nefc; r += 32) {
-          const T ja = ROW(rowJar, r), jvr = ROW(rowJv, r);
-          const T x = ja + an * jvr;
-          if (x < 0 || r < ne) {
-            const T Dx = ROW(rowD, r) * x, Dj = ROW(rowD, r) * jvr;
-            c += (T)0.5 * Dx * x;
-            d0 += Dx * jvr;
-            d1 += Dj * jvr;
-            s0 += ox_abs(Dx * jvr);
-          }
-        }
-        cur_a = an;
-        cur_c = an * an * qg2 + an * qg1 + gauss + wsum(c);
-        cur_d0 = 2 * an * qg2 + qg1 + wsum(d0);
-        cur_d1 = 2 * qg2 + wsum(d1);
-        const T cur_s0 = ox_abs(2 * an * qg2) + ox_abs(qg1) + wsum(s0);
-        if (cur_d1 < (T)OX_MINVAL) cur_d1 = (T)OX_MINVAL;
-        if (it < 0) {
-          p0c = cur_c; p0d0 = cur_d0;
-          if (!(p0d0 < 0)) stop = true;
-        } else {
-          if (ox_abs(cur_d0) < gtol || ox_abs(cur_d0) <= 8 * Eps<T>::v() * cur_s0) break;
-          if (cur_d0 < 0) lo_a = cur_a; else { hi_a = cur_a; have_hi = true; }
-        }
-      }
-      if (stop) break;
-      const T alpha = cur_c <= p0c ? cur_a : (T)0;
-      if (alpha == 0) break;
-      a += alpha * search;
-      Ma += alpha * Mv;
-      for (int r = lane; r < nefc; r += 32) ROW(rowJar, r) += alpha * ROW(rowJv, r);
-      __syncwarp();
-    }
-    const T oldcost = cost;
-    // ---- efc_force, qfrc_constraint, cost at (a, Ma, jar)
-    {
-      T crow = 0;
-      for (int r = lane; r < nefc; r += 32) {
-        const T ja = ROW(rowJar, r);
-        T f = 0;
-        if (ja < 0 || r < ne) { f = -ROW(rowD, r) * ja; crow += (T)0.5 * ROW(rowD, r) * ja * ja; }
-        ROW(rowF, r) = f;
-      }
-      __syncwarp();
-      fc = 0;
-      for (int r = 0; r < nefc; r++) {
-        const T f = ROW(rowF, r);
-        if (f != 0 && me) fc += Jat(r, lane) * f;
-      }
-      gauss = wsum(me ? (T)0.5 * (Ma - fs) * (a - as) : (T)0);
-      cost = wsum(crow) + gauss;
-    }
-    // ---- gradient, H = M + J' D_active J (row `lane` in shared memory), Cholesky, Mgrad = H^-1 grad
-    {
-      grad = me ? Ma - fs - fc : (T)0;
-      gnorm = ox_sqrt(wsum(grad * grad));
-      // row `lane` of H accumulates in registers (static indices: the j loops are fully unrolled, the row loop is not)
-      T Hreg[32];
-#pragma unroll
-      for (int j = 0; j < 32; j++) Hreg[j] = Mrow[j];
-      for (int r = 0; r < nefc; r++) {
-        if (!(ROW(rowJar, r) < 0 || r < ne)) continue;  // warp-uniform
-        if (r < COOP_SROWS) {
-          const T* jr = sJ + r * 33;  // padding columns nv..31 are zero
-          const T s = ROW(rowD, r) * jr[lane];
-#pragma unroll
-          for (int j = 0; j < 32; j++) Hreg[j] += s * jr[j];  // broadcast reads
-        } else {
-          const T Jri = me ? GA(efc_J, r * nv + lane) : (T)0;
-          const T s = ROW(rowD, r) * Jri;
-#pragma unroll
-          for (int j = 0; j < 32; j++) Hreg[j] += s * bcast(Jri, j);
-        }
-      }
-      // right-looking Cholesky on the register rows: at step kk lane i >= kk turns H[i][kk] into L[i][kk] and every lane
-      // subtracts L[i][kk] * L[j][kk] (lane j's value, one shuffle) from H[i][j]. Entries above the diagonal and the rows
-      // of idle lanes hold finite garbage that is never read.
-      T dinv = 1;
-#pragma unroll
-      for (int kk = 0; kk < 32; kk++) {
-        if (kk < nv) {  // warp-uniform
-          const T piv = bcast(Hreg[kk], kk);
-          const T inv = coop_rsqrt(ox_max(piv, (T)OX_MINVAL));  // 1 / L[kk][kk]; the diagonal itself is never needed
-          const T lik = Hreg[kk] * inv;
-          Hreg[kk] = lik;
-          if (lane == kk) dinv = inv;
-#pragma unroll
-          for (int j = kk + 1; j < 32; j++) Hreg[j] -= lik * bcast(lik, j);
-        }
-      }
-      T acc = grad, y = 0;
-#pragma unroll
-      for (int kk = 0; kk < 32; kk++) {  // L y = grad, column-oriented
-        if (kk < nv) {
-          const T yk = bcast(acc * dinv, kk);
-          if (lane == kk) y = yk;
-          if (lane > kk) acc -= Hreg[kk] * yk;
-        }
-      }
-      // L' x = y, column-oriented: lane j needs L[kk][j], which sits in lane kk's register j - so the factor goes through
-      // shared memory once (row kk contiguous: conflict-free reads) instead of 27 butterfly reductions
-#pragma unroll
-      for (int j = 0; j < 32; j++) sL[lane * 33 + j] = Hreg[j];
-      __syncwarp();
-      T x = 0;
-      acc = y;
-      for (int kk = nv - 1; kk >= 0; kk--) {
-        const T xk = bcast(acc * dinv, kk);
-        if (lane == kk) x = xk;
-        if (lane < kk) acc -= sL[kk * 33 + lane] * xk;
-      }
-      __syncwarp();
-      Mgrad = x;
-    }
-    if (init) {
-      init = false;
-      if (scale * gnorm < tol) break;
-    } else {
-      iter++;
-      const T improvement = scale * (oldcost - cost), gradient = scale * gnorm;
-      if (improvement < tol || gradient < tol) break;
-      if (oldcost - cost <= OX_FLOOR_MULT * Eps<T>::v() * (ox_abs(oldcost) + ox_abs(cost))) break;
-    }
-    search = -Mgrad;
-  }
-  if (me) { GA(qacc, lane) = a; GA(qacc_warmstart, lane) = a; GA(qfrc_constraint, lane) = fc; }
-  if (small)
-    for (int r = lane; r < nefc; r += 32) GA(efc_force, r) = ROW(rowF, r);
-  if (lane == 0) b.solver_niter[ue] = iter;
-#undef GA
-#undef ROW
-}
 
 // PERSISTENT launch: the grid holds as many CTAs as the device keeps resident; every warp draws its next environment from a
 // global ticket counter. Solve times vary several-fold between envs (0 .. 8 Newton iterations, 0 .. 90 rows), and with the
@@ -303,18 +25,17 @@ __global__ void __launch_bounds__(32 * COOP_WARPS) k_solve_coop(const unsigned c
   DevModel<T> m{stage_model(gblob, bytes)};
   extern __shared__ __align__(128) unsigned char ox_smem[];
   const int wib = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  if (!ctr) {   // static map (OX_B200_COOP_STATIC=1, kept for A/B measurements): warp w of CTA c solves env 8 c + w
-    const int env = blockIdx.x * COOP_WARPS + wib;
-    if (env < b.nenv) coop_solve_env<T>(m, b, ox_smem, bytes, env, wib, lane);
-    return;
-  }
+  T* srow = reinterpret_cast<T*>(ox_smem + ((bytes + 127) / 128) * 128) + (size_t)wib * coop_warp_words();
+  T* sJ = srow + 5 * COOP_RCAP;
+  T* sL = sJ + COOP_SROWS * 33;
+  const LaneGroup<32> g{lane, 0xffffffffu};
   for (;;) {
     int env = 0;
     if (lane == 0) env = atomicAdd(&ctr[0], 1);
     env = __shfl_sync(0xffffffffu, env, 0);
     if (env >= b.nenv) break;
-    coop_solve_env<T>(m, b, ox_smem, bytes, env, wib, lane);
-    __syncwarp();   // the warp's shared-memory scratch is reused by its next environment
+    // ends with a warp sync: the warp's shared-memory scratch is then free for its next environment
+    group_newton<T, 32, COOP_RCAP>(g, m, b, ElemAt{(uint32_t)b.stride, (uint32_t)env}, sJ, sL, srow);
   }
   if (lane == 0) {
     const int done = atomicAdd(&ctr[1], 1);
@@ -351,9 +72,7 @@ template <typename T>
 static cudaError_t launch_coop(cudaStream_t stream, const unsigned char* blob, int bytes, const DevBatch<T>& b, int resident_ctas, int* ctr) {
   const size_t smem = solve_coop_smem(bytes, sizeof(T) == 8);
   int grid = (b.nenv + COOP_WARPS - 1) / COOP_WARPS;
-  static const bool force_static = [] { const char* e = getenv("OX_B200_COOP_STATIC"); return e && *e == '1'; }();
-  if (force_static) ctr = nullptr;
-  else if (resident_ctas > 0 && grid > resident_ctas) grid = resident_ctas;
+  if (resident_ctas > 0 && grid > resident_ctas) grid = resident_ctas;
   k_solve_coop<T><<<grid, 32 * COOP_WARPS, smem, stream>>>(blob, bytes, b, ctr);
   return cudaPeekAtLastError();  // the caller propagates it (CU_TRY); peek so that the sticky state is not silently cleared
 }
