@@ -10,6 +10,7 @@
  *   ox_batch_create             <- mj_makeData              src/physics.rs:14,22  (batched: nenv copies of mjData, SoA on device)
  *   ox_batch_step               <- Physics::step            src/physics.rs:44-46  (mj_step)      ** the hot path **
  *   ox_batch_forward            <- Physics::forward         src/physics.rs:48-50  (mj_forward)
+ *   ox_batch_inverse            <- (extension)              mj_inverse, batched
  *   ox_batch_reset              <- Physics::reset           src/physics.rs:52-54  (mj_resetData, masked)
  *   ox_model_name2id/id2name    <- object_id / object_name  src/physics.rs:56-62
  *   ox_batch_set1/get1, set/get <- Actuators::set, time/ctrl/act/qpos/qvel/qacc_warmstart/qfrc_applied/
@@ -234,6 +235,17 @@ OX_API void* ox_batch_stream(const ox_batch* b); /* cudaStream_t */
 /* step family: asynchronous on the batch's stream */
 OX_API ox_status ox_batch_step(ox_batch* b, int32_t nsteps);
 OX_API ox_status ox_batch_forward(ox_batch* b);
+/* Inverse dynamics (mj_inverse, continuous time) of every env, one launch on the batch's stream. From qpos, qvel, qacc,
+ * ctrl, act, mocap, eq_active and the applied forces it writes
+ *   qfrc_inverse = M(qpos) qacc + qfrc_bias - qfrc_passive - qfrc_constraint,   qfrc_constraint = J' efc_force,
+ * where efc_force is the soft-constraint force at J qacc - aref (mj_invConstraint): the same function for PGS, CG and Newton
+ * models, noslip not applied. It also writes every position- and velocity-dependent field ox_batch_forward writes (kinematics,
+ * qM / qLD, bias, passive, tendons, contacts, constraint rows with the inverse efc_force and qfrc_constraint), the actuation
+ * fields actuator_force / qfrc_actuator / act_dot, qfrc_smooth / qacc_smooth (which mj_inverse leaves stale), and sensordata
+ * computed with the given qacc. Afterwards every derived field is readable. It never writes qpos, qvel, qacc,
+ * qacc_warmstart, ctrl, act, time, the applied forces, mocap, eq_active, solver_niter, diverged, the statistics or the Philox
+ * step counter; there is no divergence check and no auto-reset. */
+OX_API ox_status ox_batch_inverse(ox_batch* b);
 /* Action::apply + Physics::step + Observation::generate of Environment::step (reference src/lib.rs:63-66) in ONE call for the
  * whole batch: ctrl[nenv][nu] in (NULL = keep), one mj_step, qpos[nenv][nq] / qvel[nenv][nv] out (either may be NULL); env-major
  * `dtype` buffers in `mem`. With a model-specialised kernel and device memory or pinned host memory the step kernel reads and
@@ -263,6 +275,7 @@ enum {
   OX_F_CON_DIST, OX_F_CON_POS, OX_F_CON_FRAME,
   OX_F_EFC_J, OX_F_EFC_POS, OX_F_EFC_MARGIN, OX_F_EFC_D, OX_F_EFC_AREF, OX_F_EFC_FORCE,
   OX_F_ACT_DOT, OX_F_MOCAP_POS, OX_F_MOCAP_QUAT, OX_F_EQ_ACTIVE, OX_F_TEN_LENGTH, OX_F_TEN_J,
+  OX_F_QFRC_INVERSE, /* written by ox_batch_inverse only; zeros until its first call */
   OX_F_COUNT_REAL,
   /* int32 fields */
   OX_F_NCON = 100, OX_F_NEFC, OX_F_SOLVER_NITER, OX_F_DIVERGED, OX_F_CON_PAIR

@@ -82,6 +82,7 @@ class BatchedPhysics {
   }
   void step(int nsteps = 1) { check(ox_batch_step(b_, nsteps)); }
   void forward() { check(ox_batch_forward(b_)); }
+  void inverse() { check(ox_batch_inverse(b_)); }   // extension: mj_inverse for every env, result in OX_F_QFRC_INVERSE
   // ctrl in, one step, qpos / qvel out in one call (Action::apply + step + Observation::generate, src/lib.rs:63-66)
   void step_io(const void* ctrl, void* qpos, void* qvel, int dtype, int mem = OX_MEM_HOST) { check(ox_batch_step_io(b_, ctrl, qpos, qvel, dtype, mem)); }
   void reset(const uint8_t* mask = nullptr) { check(ox_batch_reset(b_, mask)); }
@@ -146,6 +147,7 @@ class Physics {
   BatchedPhysics& data_mut() { return batch_; }                                                                  // :33-35
   void step() { batch_.step(1); batch_.sync(); }                                                                 // :44-46
   void forward() { batch_.forward(); batch_.sync(); }                                                            // :48-50
+  void inverse() { batch_.inverse(); batch_.sync(); }                                                            // extension: mj_inverse
   void reset() { batch_.reset(); batch_.sync(); }                                                                // :52-54
   template <int O> std::optional<ObjectId<O>> object_id(const std::string& n) const { return model_.object_id<O>(n); }
   template <int O> std::string object_name(ObjectId<O> id) const { return model_.object_name(id); }

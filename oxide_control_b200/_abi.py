@@ -31,7 +31,7 @@ _REAL_FIELDS = [
     "site_xpos", "site_xmat", "subtree_com", "cinert", "cdof", "qM", "qLD", "qLDiagInv", "cvel", "cdof_dot",
     "qfrc_bias", "qfrc_passive", "actuator_force", "qfrc_actuator", "qfrc_smooth", "qacc_smooth", "qfrc_constraint",
     "con_dist", "con_pos", "con_frame", "efc_J", "efc_pos", "efc_margin", "efc_D", "efc_aref", "efc_force", "act_dot",
-    "mocap_pos", "mocap_quat", "eq_active", "ten_length", "ten_J",
+    "mocap_pos", "mocap_quat", "eq_active", "ten_length", "ten_J", "qfrc_inverse",
 ]
 FIELD = {name: i for i, name in enumerate(_REAL_FIELDS)}
 FIELD.update({"ncon": 100, "nefc": 101, "solver_niter": 102, "diverged": 103, "con_pair": 104})
@@ -95,6 +95,7 @@ SYMBOLS = {
     "ox_batch_stream": (_P, [_P]),
     "ox_batch_step": (C.c_int32, [_P, C.c_int32]),
     "ox_batch_forward": (C.c_int32, [_P]),
+    "ox_batch_inverse": (C.c_int32, [_P]),
     "ox_batch_step_io": (C.c_int32, [_P, _P, _P, _P, C.c_int32, C.c_int32]),
     "ox_batch_reset": (C.c_int32, [_P, _P]),
     "ox_batch_sync": (C.c_int32, [_P]),

@@ -37,6 +37,9 @@ size_t layout_arena(const ox_model_tables& t, int stride, unsigned char* base, D
   }
   OX_BATCH_INT_FIELDS(OX_X)
 #undef OX_X
+  // qfrc_inverse (ox_batch_inverse): appended after every DevBatch field and kept out of DevBatch, whose size and field
+  // lists fix the shared-memory and per-thread layouts of the step kernels; k_inverse receives the pointer as an argument
+  const size_t off_inverse = take((size_t)nv, sizeof(T));
   if (out && fields) {
     auto& f = *fields;
 #define R(id, name, cnt) f[id] = FieldInfo{out->name, (int)(cnt), false};
@@ -56,6 +59,7 @@ size_t layout_arena(const ox_model_tables& t, int stride, unsigned char* base, D
     R(OX_F_ACT, act, na) R(OX_F_ACT_DOT, act_dot, na) R(OX_F_MOCAP_POS, mocap_pos, 3 * nmc) R(OX_F_MOCAP_QUAT, mocap_quat, 4 * nmc)
     R(OX_F_EQ_ACTIVE, eq_active, neq) R(OX_F_TEN_LENGTH, ten_length, nten) R(OX_F_TEN_J, ten_J, nten * nv)
 #undef R
+    f[OX_F_QFRC_INVERSE] = FieldInfo{base + off_inverse, (int)nv, false};
 #define I(id, name, cnt) f[id] = FieldInfo{out->name, (int)(cnt), true};
     I(OX_F_NCON, ncon, 1) I(OX_F_NEFC, nefc, 1) I(OX_F_SOLVER_NITER, solver_niter, 1) I(OX_F_DIVERGED, diverged, 1)
     I(OX_F_CON_PAIR, con_pair, ncm)

@@ -66,6 +66,7 @@ inline bool field_live(bool stale, bool split, int field) {
     case OX_F_QPOS: case OX_F_QVEL: case OX_F_CTRL: case OX_F_QFRC_APPLIED: case OX_F_XFRC_APPLIED: case OX_F_QACC_WARMSTART:
     case OX_F_TIME: case OX_F_ACT: case OX_F_ACT_DOT: case OX_F_QACC: case OX_F_SENSORDATA: case OX_F_NCON: case OX_F_NEFC: case OX_F_SOLVER_NITER:
     case OX_F_DIVERGED: case OX_F_MOCAP_POS: case OX_F_MOCAP_QUAT: case OX_F_EQ_ACTIVE:
+    case OX_F_QFRC_INVERSE:   // no step writes it: it holds what the last ox_batch_inverse wrote
       return true;
     case OX_F_QM: case OX_F_QFRC_SMOOTH: case OX_F_QACC_SMOOTH: case OX_F_QFRC_CONSTRAINT: case OX_F_EFC_J: case OX_F_EFC_POS:
     case OX_F_EFC_MARGIN: case OX_F_EFC_D: case OX_F_EFC_AREF: case OX_F_EFC_FORCE:

@@ -253,6 +253,11 @@ class BatchedPhysics:
     def forward(self) -> None:
         _check(A.lib().ox_batch_forward(self._h))
 
+    def inverse(self) -> None:
+        """mj_inverse for every env (ox_batch_inverse): qfrc_inverse = M qacc + bias - passive - constraint at the current
+        qpos / qvel / qacc, plus every derived field and sensordata. The state and qacc are left as they are."""
+        _check(A.lib().ox_batch_inverse(self._h))
+
     def step_io(self, ctrl: Optional[np.ndarray] = None):
         """Action::apply + step + Observation::generate (src/lib.rs:63-66) for the whole batch in one call:
         ctrl[nenv, nu] in, one mj_step, (qpos[nenv, nq], qvel[nenv, nv]) out."""
@@ -542,6 +547,11 @@ class Physics:
 
     def forward(self) -> None:
         self._b.forward()
+        self._b.sync()
+
+    # extension: mj_inverse; the result is data().qfrc_inverse
+    def inverse(self) -> None:
+        self._b.inverse()
         self._b.sync()
 
     def reset(self) -> None:

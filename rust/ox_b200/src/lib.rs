@@ -173,6 +173,8 @@ impl BatchedPhysics {
     pub fn kernel_name(&self) -> String { unsafe { CStr::from_ptr(sys::ox_batch_kernel_name(self.raw)).to_string_lossy().into_owned() } }
     pub fn step(&mut self, nsteps: i32) { let _ = unsafe { sys::ox_batch_step(self.raw, nsteps) }; }     // infallible like src/physics.rs:44
     pub fn forward(&mut self) { let _ = unsafe { sys::ox_batch_forward(self.raw) }; }
+    /// extension: mj_inverse for every env; the result is the field `OX_F_QFRC_INVERSE` (infallible like `forward`)
+    pub fn inverse(&mut self) { let _ = unsafe { sys::ox_batch_inverse(self.raw) }; }
     pub fn reset(&mut self, mask: Option<&[u8]>) { let _ = unsafe { sys::ox_batch_reset(self.raw, mask.map_or(std::ptr::null(), |m| m.as_ptr())) }; }
     pub fn sync(&self) -> Result<(), Error> { check(unsafe { sys::ox_batch_sync(self.raw) }) }
     /// controls in, one step, qpos / qvel out in one call (Action::apply + step + Observation::generate, src/lib.rs:63-66)
@@ -267,6 +269,8 @@ impl Physics {
 
     pub fn step(&mut self) { self.data.step(1); let _ = self.data.sync(); }         // :44-46  mj_step
     pub fn forward(&mut self) { self.data.forward(); let _ = self.data.sync(); }    // :48-50  mj_forward
+    /// extension (no counterpart in the reference): mj_inverse; read `OX_F_QFRC_INVERSE` through `data()`
+    pub fn inverse(&mut self) { self.data.inverse(); let _ = self.data.sync(); }
     pub fn reset(&mut self) { self.data.reset(None); let _ = self.data.sync(); }    // :52-54  mj_resetData
 
     pub fn object_id<O: Obj>(&self, name: &str) -> Option<ObjectId<O>> { self.model.object_id(name) }    // :56-58
